@@ -24,6 +24,13 @@ A "step" is one createIndex over the whole table: scan (Parquet decode) -> proje
                 image), so this arm times the oracle port with all host threads, as the task statement prescribes.
 * ``extra``     the read-side and refresh workloads of BASELINE.json configs[2..4] (C3 filter, C4 join, C5 incremental
                 refresh + Hybrid Scan), each runnable alone with ``--workload``.
+* ``--dump-outputs DIR``  after the timed steps, a seeded sample of the index files of the last timed step as
+                DIR/<name>.npy (see dump_outputs), the same for the same arguments, to compare two builds output for output.
+                That step's index files stay in HBM until the dump is written, so its release (hs_result_free, a stream
+                synchronize) falls outside the timed region: compare timings of dump runs with dump runs only.
+
+Every workload (and the reference arm) runs ``--warmup`` untimed and ``--steps`` timed repetitions, except that the
+pipelined e2e path always warms up at least two steps and the ``cpu_baseline`` is a fixed best of 3 after one warm-up.
 
 Multi-GPU (torchrun, one rank per GPU): the 256 source files are split across ranks, rows move to the owner of their
 bucket inside the fused partition + NVLink peer-store kernel, the table size is fixed (strong scaling).
@@ -76,7 +83,14 @@ def parse_args():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the C3/C4/C5 workloads attached under 'extra'")
     ap.add_argument("--plain", action="store_true", help="PLAIN-only source and index files (no dictionary encoding)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed, seeded sample of the index rows of the last timed createIndex step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "createIndex"):
+        ap.error("--dump-outputs needs the createIndex workload on the GPU")
+    return args
 
 
 class ClockSampler:
@@ -213,13 +227,13 @@ def run_reference(args):
         return
     from oracle import oracle as O
 
-    O.build()
+    O.lib()  # built by __graft_entry__.build(); no staleness rebuild here, as the tree may be read-only
     cores = os.cpu_count() or 1
     rows, files = args.cpu_sample_rows, args.cpu_sample_files
     rows = rows // files * files
     with tempfile.TemporaryDirectory() as wd:
         paths = cpu_write_sources(rows, files, cores, wd)
-        for _ in range(max(1, min(args.warmup, 1))):
+        for _ in range(args.warmup):
             cpu_create_index(paths, cores, wd)
         times = [cpu_create_index(paths, cores, wd) for _ in range(args.steps)]
     sec = sum(times) / len(times)
@@ -404,7 +418,7 @@ def verify_output(rig, res, first_row, my_rows, total_rows, what):
 
         from oracle import oracle as O
 
-        O.build()
+        O.lib()  # built by __graft_entry__.build(); no staleness rebuild here, as the tree may be read-only
         t1 = time.perf_counter()
         oracle_ok = True
         for i in sorted({0, len(res.files) - 1}):
@@ -428,6 +442,73 @@ def verify_output(rig, res, first_row, my_rows, total_rows, what):
     return verified, all_ok
 
 
+DUMP_SAMPLE_ROWS = 1 << 19  # index rows written by --dump-outputs over all buckets (~36 MB of .npy files)
+DUMP_SEED = 20201017
+
+
+def _float_columns(name, a):
+    """A column as float arrays that hold it exactly: int64 as its high (signed) and low 32 bits, int32 and float64 as
+    float64, float32 as is."""
+    import numpy as np
+
+    if a.dtype == np.int64:
+        return {f"{name}_hi": (a >> 32).astype(np.float64), f"{name}_lo": (a & 0xFFFFFFFF).astype(np.float64)}
+    if a.dtype == np.float32:
+        return {name: a}
+    return {name: a.astype(np.float64)}
+
+
+def dump_outputs(rig, res, out_dir):
+    """Writes what a caller of createIndex receives, for comparing two builds output for output: the row count of every
+    bucket file, and for a seeded sample of positions inside every bucket file (the same positions whenever the bucket
+    holds the same number of rows) the bucket, the position and every column of the rows found there.  `res` holds
+    this rank's index files in HBM; rank 0 writes DIR/<name>.npy.  Returns what was written (rank 0)."""
+    import types
+    from concurrent.futures import ThreadPoolExecutor
+
+    import numpy as np
+    import pyarrow as pa
+    import pyarrow.parquet as pq
+
+    torch = rig.torch
+    device = torch.device("cuda", rig.local_rank)
+    per_bucket = max(1, DUMP_SAMPLE_ROWS // NUM_BUCKETS)
+
+    def sample(f):
+        # the engine's device allocation, wrapped by torch without a copy, then copied to the host
+        cai = {"shape": (f.size,), "typestr": "|u1", "data": (f.ptr, False), "version": 3}
+        # (worker threads start on device 0: name this rank's device, or the image would travel through GPU 0)
+        image = torch.as_tensor(types.SimpleNamespace(__cuda_array_interface__=cai), device=device).cpu().numpy()
+        t = pq.ParquetFile(pa.BufferReader(image)).read(columns=INDEXED + INCLUDED)
+        rng = np.random.default_rng([DUMP_SEED, f.bucket])
+        pos = np.sort(rng.choice(t.num_rows, size=min(per_bucket, t.num_rows), replace=False))
+        rows = t.take(pa.array(pos))
+        cols = {"bucket": np.full(len(pos), f.bucket, dtype=np.float64), "position": pos.astype(np.float64)}
+        for c in INDEXED + INCLUDED:
+            cols.update(_float_columns(c, rows.column(c).to_numpy()))
+        return f.bucket, t.num_rows, cols
+
+    with ThreadPoolExecutor(max_workers=min(16, os.cpu_count() or 1)) as ex:
+        mine = list(ex.map(sample, res.files))
+    everything = sorted((s for part in rig.gather_objects(mine) for s in part), key=lambda s: s[0])
+    if rig.rank != 0:
+        return None
+    bucket_rows = np.zeros(NUM_BUCKETS, dtype=np.float64)
+    for b, n, _ in everything:
+        bucket_rows[b] = n
+    arrays = {"bucket_rows": bucket_rows}
+    for name in everything[0][2] if everything else ():
+        arrays[name] = np.concatenate([cols[name] for _, _, cols in everything])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    return {"dir": out_dir, "arrays": sorted(arrays), "rows_sampled": int(len(arrays.get("bucket", ()))),
+            "bytes": int(sum(a.nbytes for a in arrays.values())),
+            "what": f"index files of the last timed step: rows of every bucket file, and at up to {per_bucket} seeded "
+                    f"positions per bucket file (seed {DUMP_SEED}) the bucket, the position and every column; int64 "
+                    "columns as <name>_hi / <name>_lo (high and low 32 bits)"}
+
+
 def run_create_index(rig, args):
     N, ctx, torch = rig.N, rig.ctx, rig.torch
     world, rank = rig.world, rig.rank
@@ -446,9 +527,14 @@ def run_create_index(rig, args):
     sources = src.as_sources()
     src_bytes = sum(f.size for f in src.files)
 
-    def step_device():
+    kept = [None]  # index files of the last timed step, left in HBM for --dump-outputs
+
+    def step_device(keep=False):
         res, st = ctx.create_index(sources, INDEXED, INCLUDED, NUM_BUCKETS, output=N.HS_OUT_DEVICE, **kw)
-        res.free()
+        if keep:
+            kept[0] = res
+        else:
+            res.free()
         return st
 
     for _ in range(args.warmup):
@@ -464,18 +550,24 @@ def run_create_index(rig, args):
 
     def timed_steps():
         nonlocal launches
-        for _ in range(args.steps):
-            st = step_device()
+        for i in range(args.steps):
+            st = step_device(keep=bool(args.dump_outputs) and i == args.steps - 1)
             launches += int(st["gpu_launches"])
             rows_out[0] = int(st["rows_out"])
             for k, v in st.items():
                 if k.startswith("ms_"):
                     stage_ms[k] = stage_ms.get(k, 0.0) + v / args.steps
 
-    ms_total, _ = rig.timed(timed_steps)
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        ms_total, _ = rig.timed(timed_steps)
+    finally:
+        clocks = sampler.stop() if rank == 0 else None  # never leave nvidia-smi running behind a failed step
     kernels = ctx.profile_report()
     ctx.profile_enable(False)
+    dumped = None
+    if args.dump_outputs:
+        dumped = dump_outputs(rig, kept[0], args.dump_outputs)
+        kept[0].free()
     ms_dev = ms_total / args.steps
     value = total_rows / (ms_dev / 1e3)
     roofline = roofline_of(kernels, args.steps, my_rows, rows_out[0] or total_rows / world, value, world)
@@ -531,14 +623,18 @@ def run_create_index(rig, args):
             res.free()
             return st
 
+        # at least two steps: a one-step warm-up never has two calls in flight, and the timed steps then pay for that
+        # set-up (e2e about 10x slower with --warmup 1 on a B200 at 1000 W)
         pipelined(max(2, args.warmup))
         for v in copy_ms.values():
             v.clear()
         ms_pipe, _ = rig.timed(lambda: pipelined(args.steps, keep_last=not args.no_verify))
         avg = lambda v: (sum(v) / len(v)) if v else None  # noqa: E731
         ms_e2e = ms_pipe / args.steps
-        single_call()
-        ms_single, st_single = rig.timed(single_call)
+        for _ in range(args.warmup):
+            single_call()
+        ms_single, st_single = rig.timed(lambda: [single_call() for _ in range(args.steps)][-1])
+        ms_single /= args.steps
         e2e = {"value": total_rows / (ms_e2e / 1e3), "unit": "rows/s", "h2d_bytes_per_step": int(src_bytes),
                "d2h_bytes_per_step": int(out_bytes[0]), "ms_per_step": ms_e2e,
                "h2d_GBps_per_rank": src_bytes / (ms_e2e / 1e3) / 1e9, "d2h_GBps_per_rank": out_bytes[0] / (ms_e2e / 1e3) / 1e9,
@@ -548,8 +644,8 @@ def run_create_index(rig, args):
                "note": "pinned HOST Parquet images in, HOST index images out, per-rank bytes; timed over K steps software-pipelined "
                        "through hs_stage_sources / hs_create_index_async / hs_pending_wait (H2D of step i+1 and D2H of step i-1 "
                        "beside the kernels of step i; every step's copies are inside the timed region, fill and drain included). "
-                       "single_call_ms = one synchronous hs_create_index (H2D, build, D2H back to back: a call cannot overlap its "
-                       "own copies because every index file depends on every source file)"}
+                       "single_call_ms = one synchronous hs_create_index, averaged over K calls (H2D, build, D2H back to back: "
+                       "a call cannot overlap its own copies because every index file depends on every source file)"}
         if not args.no_verify:
             verified, verified_ok = verify_output(rig, last[0], first_row, my_rows, total_rows,
                                                   "index files of the last timed e2e step (host images)")
@@ -570,6 +666,8 @@ def run_create_index(rig, args):
         "clocks": clocks, "e2e": e2e, "gpu_launches": launches, "roofline": roofline, "verified": verified,
         "stage_ms_per_step": stage_ms,
     }
+    if dumped:
+        line["dump_outputs"] = dumped
     return line, verified_ok
 
 
@@ -596,7 +694,7 @@ def run_ours(args):
         try:
             from oracle import oracle as O
 
-            O.build()
+            O.lib()  # built by __graft_entry__.build(); no staleness rebuild here, as the tree may be read-only
             cores = os.cpu_count() or 1
             files = args.cpu_sample_files
             rows = args.cpu_sample_rows // files * files

@@ -6,7 +6,7 @@ Sizes follow SURVEY.md section 8d, scaled from ``--rows`` (1 B by default):
   C3  FilterIndexRule scan (index/covering/FilterIndexRule.scala:135-149): ``k BETWEEN lo AND hi`` covering 1 % of the int64
       key space over the rows-row / 200-bucket index, projecting k, v1, v2 (~rows/100 rows out), 20 distinct ranges.
       Buckets are owner-sharded (bucket b lives on GPU b mod N, where createIndex wrote it): every rank scans its own files,
-      no collective.  queries/s = 20 / time (max over ranks).
+      no collective.  A step is one pass over the 20 ranges; queries/s = 20 x steps / time (max over ranks).
   C4  JoinIndexRule bucket-aligned merge join (index/covering/JoinIndexRule.scala:653-687): L = rows/2 rows with
       k = splitmix64(42, i); R = rows/2 rows whose keys are those of the first rows/4 rows of T, each twice => rows/2 matches,
       half of L unmatched.  ``SELECT L.v1, R.v2``.  Bucket b of L and of R sit on the same GPU by construction: no collective.
@@ -16,6 +16,7 @@ Sizes follow SURVEY.md section 8d, scaled from ``--rows`` (1 B by default):
       join = appended rows bucketed on the fly + merge join over buckets that now hold two files.
 
 Every number carries its algorithmic bytes (SURVEY.md 8d "read side") and the achieved fraction of the HBM peak.
+Every timed loop runs ``--warmup`` untimed repetitions and then ``--steps`` timed ones.
 Index files stay resident in HBM (the index of a running cluster is hot in the scan cache); results are produced both
 into pinned host memory (D2H inside the timed region) and left on the device for the next GPU operator.
 """
@@ -95,25 +96,29 @@ def run_filter(rig, args, idx=None, appended=None):
             return n, st
 
         rs = _ranges(QUERIES)
-        one(*rs[0])  # warm
+        for _ in range(args.warmup):
+            for lo, hi in rs:
+                one(lo, hi)
         rows_out = [0]
         last = [None]
 
         def timed():
-            for lo, hi in rs:
-                n, st = one(lo, hi)
-                rows_out[0] += n
-                last[0] = st
+            for _ in range(args.steps):
+                for lo, hi in rs:
+                    n, st = one(lo, hi)
+                    rows_out[0] += n
+                    last[0] = st
 
         ms, _ = rig.timed(timed)
+        nq = QUERIES * args.steps
         total_out = _sum_over_ranks(rig, rows_out[0])
         sec = ms / 1e3
-        per_q = total_out / QUERIES
+        per_q = total_out / nq
         algo = per_q * 48.0  # 24 B read + 24 B written per qualifying row (SURVEY.md 8d); the probes are negligible
-        out[mode] = {"queries_per_s": QUERIES / sec, "ms_per_query": ms / QUERIES, "rows_out_per_query": per_q,
+        out[mode] = {"queries_per_s": nq / sec, "ms_per_query": ms / nq, "rows_out_per_query": per_q,
                      "rows_out_per_s": total_out / sec, "algorithmic_GB_per_query": algo / 1e9,
-                     "achieved_GBps_per_gpu": algo / (ms / QUERIES / 1e3) / 1e9 / rig.world,
-                     "frac_of_hbm_peak": algo / (ms / QUERIES / 1e3) / 1e9 / rig.world / _peak()}
+                     "achieved_GBps_per_gpu": algo / (ms / nq / 1e3) / 1e9 / rig.world,
+                     "frac_of_hbm_peak": algo / (ms / nq / 1e3) / 1e9 / rig.world / _peak()}
     # cross-check of one query: the indexed answer has as many rows as a full predicate scan of the same files
     lo, hi = _ranges(1)[0]
     a, _ = ctx.filter_scan(files, "k", ["k"], lo=lo, hi=hi, output=N.HS_OUT_DEVICE)
@@ -125,7 +130,7 @@ def run_filter(rig, args, idx=None, appended=None):
         idx.free()
         ctx.trim()
     res = {"workload": f"C3: k BETWEEN lo AND hi (1% of the key space) over the {args.rows}-row {NB}-bucket index, project k,v1,v2; "
-                       f"{QUERIES} ranges; buckets owner-sharded over {rig.world} GPU(s), no collective; index resident in HBM",
+                       f"{QUERIES} ranges per step; buckets owner-sharded over {rig.world} GPU(s), no collective; index resident in HBM",
            "result_to_host": out["host"], "result_on_device": out["device"],
            "checked": {"indexed_rows == full_scan_rows": bool(same)}}
     if appended:
@@ -153,16 +158,16 @@ def run_join(rig, args):
             b.free()
             return n, st
 
-        one()
-        reps = 3
+        for _ in range(args.warmup):
+            one()
         acc = [0, None]
 
         def timed():
-            for _ in range(reps):
+            for _ in range(args.steps):
                 acc[0], acc[1] = one()
 
         ms, _ = rig.timed(timed)
-        ms /= reps
+        ms /= args.steps
         nout_total = _sum_over_ranks(rig, acc[0])
         algo = 16.0 * jr + 16.0 * jr + 16.0 * nout_total  # (k + payload) of both sides read once, 16 B per output row written
         out[mode] = {"joins_per_s": 1e3 / ms, "ms_per_join": ms, "rows_out": nout_total, "rows_out_per_s": nout_total / (ms / 1e3),
@@ -202,21 +207,21 @@ def run_refresh(rig, args):
                                    save_mode=N.HS_SAVE_APPEND)
         return res, st
 
-    r, _ = refresh()
-    r.free()
-    reps = 3
+    for _ in range(args.warmup):
+        r, _ = refresh()
+        r.free()
     keep = [None]
 
     def timed():
-        for i in range(reps):
+        for i in range(args.steps):
             res, st = refresh()
-            if i == reps - 1:
+            if i == args.steps - 1:
                 keep[0] = (res, st)
             else:
                 res.free()
 
     ms, _ = rig.timed(timed)
-    ms /= reps
+    ms /= args.steps
     inc, st = keep[0]
     rep = ctx.verify_index(inc.as_sources(), [f.bucket for f in inc.files], ["k"], ["v1", "v2", "v3", "v4"], NB)
     gen = ctx.synth_checksum(fr, my_rows, 5)
@@ -246,13 +251,16 @@ def run_refresh(rig, args):
         tmp.free()
         return n, stj
 
-    hybrid_join(N.HS_OUT_DEVICE)
+    for _ in range(args.warmup):
+        hybrid_join(N.HS_OUT_DEVICE)
     acc = [0]
 
     def timed_join():
-        acc[0], _ = hybrid_join(N.HS_OUT_DEVICE)
+        for _ in range(args.steps):
+            acc[0], _ = hybrid_join(N.HS_OUT_DEVICE)
 
     msj, _ = rig.timed(timed_join)
+    msj /= args.steps
     nout = _sum_over_ranks(rig, acc[0])
     hyb_join = {"ms": msj, "rows_out": nout, "checked": {"matches == delta_rows": bool(int(nout) == total_delta)},
                 "what": f"({rows}-row index U {total_delta} appended rows bucketed on the fly) JOIN ({total_delta}-row index) ON k; "
@@ -282,18 +290,18 @@ def run_snappy(rig, args):
             nbytes = sum(f.size for f in res.files)
             res.free()
             return st, nbytes
-        one()
-        one()
+        for _ in range(args.warmup):
+            one()
         ctx.profile_enable(True)
         acc = [None, 0]
 
         def loop():
-            for _ in range(3):
+            for _ in range(args.steps):
                 acc[0], acc[1] = one()
         ms, _ = rig.timed(loop)
         kernels = ctx.profile_report()
         ctx.profile_enable(False)
-        return ms / 3, {k: v["ms"] / 3 for k, v in kernels.items()}, acc[1]
+        return ms / args.steps, {k: v["ms"] / args.steps for k, v in kernels.items()}, acc[1]
 
     usrc = ctx.synth_table(fr, my_rows, 5, n_files=max(1, my_files), row_groups_per_file=4, output=N.HS_OUT_DEVICE)
     ms_u, k_u, bytes_u = timed_builds(usrc.as_sources())
@@ -331,8 +339,9 @@ def run_snappy(rig, args):
 def run_files(rig, args):
     """The reference's actual effect: Parquet files in, bucket files out (index/DataFrameWriterExtensions.scala:50-68 writes
     them under <index>/v__=N).  createIndex with path sources and HS_OUT_FILES: file reads (a few host threads into pinned
-    memory), H2D, build, D2H, file writes (a few host threads) -- one blocking call, nothing pipelined.  tmpfs and, where a
-    writable disk with room exists, the local file system; a quarter of --rows to keep the run short."""
+    memory), H2D, build, D2H, file writes (a few host threads) -- one blocking call, nothing pipelined; the best of --steps
+    calls after --warmup untimed ones.  tmpfs and, where a writable disk with room exists, the local file system; a quarter
+    of --rows to keep the run short."""
     import shutil
     import tempfile
     import time
@@ -363,8 +372,10 @@ def run_files(rig, args):
                     fh.write(src.host_bytes(i))
                 paths.append(p)
             files = [N.FileImage(path=p, file_id=i) for i, p in enumerate(paths)]
-            best, stats = None, None
-            for rep in range(3):
+            best, stats, out_dir = None, None, None
+            for rep in range(args.warmup + args.steps):
+                if out_dir:
+                    shutil.rmtree(out_dir)  # keep one call's output at a time: the room needed does not grow with --steps
                 out_dir = os.path.join(root, f"v__={rep}")
                 t0 = time.perf_counter()
                 res, st = ctx.create_index(files, ["k"], ["v1", "v2", "v3", "v4"], NB, out_dir=out_dir, output=N.HS_OUT_FILES,
@@ -372,13 +383,14 @@ def run_files(rig, args):
                 dt = time.perf_counter() - t0
                 n_out = len(res.files)
                 res.free()
-                if rep and (best is None or dt < best):
+                if rep >= args.warmup and (best is None or dt < best):
                     best, stats = dt, st
             idx_bytes = sum(os.path.getsize(os.path.join(out_dir, n)) for n in os.listdir(out_dir) if n.endswith(".parquet"))
             out[label] = {"rows_per_s": rows / best, "ms": best * 1e3, "index_files": n_out, "index_bytes": idx_bytes,
                           "GBps_in_plus_out": (src_bytes + idx_bytes) / best / 1e9,
                           "stage_ms": {k: round(v, 2) for k, v in stats.items() if k.startswith("ms_")},
-                          "note": "wall clock of the call, best of 2 after one warm-up; files come from / go to the page cache"}
+                          "note": f"wall clock of the call, best of {args.steps} after {args.warmup} warm-up call(s); files come from / "
+                                  "go to the page cache"}
         except Exception as ex:
             out[label] = {"failed": f"{type(ex).__name__}: {ex}"}
         finally:
